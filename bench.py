@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """PPO-update throughput of the B200 path (BASELINE.json metric: graph-samples/s + achieved HBM GB/s vs roofline).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A "step" is one PPO minibatch update -- forward + backward of the SGNN policy/value net on 256 rollout graphs per
 GPU, gradient reduction, (N>1: NCCL all-reduce of the 55 KB gradient buffer), clip + Adam -- on synthetic
@@ -90,6 +90,18 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+def dump_outputs(out_dir: str, params, grad, losses):
+    """One timed step's results as float32 .npy files: the parameters after the step, the gradient, the loss
+    statistics [0..7] of the gradient buffer (include/upb200.h) and the four logged losses."""
+    from drl_urban_planning_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    g = grad.cpu().numpy()
+    arrays = {"params": params.cpu().numpy(), "grad": g[:_lib.UPB_NUM_PARAMS],
+              "grad_stats": g[_lib.UPB_STAT_OFFSET:_lib.UPB_STAT_OFFSET + 8], "losses": np.asarray(losses)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def workload_name(args):
     return "+".join(args.mixed.split(",")) + " mixed" if args.mixed else args.community
 
@@ -137,8 +149,8 @@ def cpu_port_step_time(states, actions, flat, steps: int, warmup: int, threads: 
 
 
 def reference_kind():
-    """"reference": the unmodified reference staged by oracle/stage_ref.py (oracle/_ref, travels to the GPU box) or
-    present at /root/reference; "port": the pinned oracle restatement of its dataflow (fallback)."""
+    """"reference": the unmodified reference staged under oracle/_ref by oracle/stage_ref.py; "port": the pinned
+    oracle restatement of its dataflow (fallback)."""
     try:
         from oracle import ref_runner
         return "reference" if ref_runner.available() else "port"
@@ -225,7 +237,13 @@ def main():
     ap.add_argument("--padded-gpu", action="store_true",
                     help="also time the padded eager PyTorch dataflow (reference layout, oracle/_ref or port) on this GPU: "
                          "the padded-layout comparator of configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step returned (parameters after the step, "
+                         "gradient, loss statistics, losses) as DIR/<name>.npy; the inputs are seeded, so two builds "
+                         "run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     args.warmup = max(args.warmup, 3)
     if args.tiles == "bf16":
         os.environ["UPB_LIB"] = os.path.join(ROOT, "drl_urban_planning_b200", "libupb200_bf16.so")
@@ -327,6 +345,8 @@ def main():
     total_ms = float(ms.item())
     launches = eng.launches - launches0
     losses = eng.read_losses(grad)          # of the last timed step
+    # what the last timed step returned, kept before the steps below move the parameters on
+    last = (params.clone(), grad.clone()) if args.dump_outputs else None
     # the timed region lasts a few ms, too short for nvidia-smi: keep the same load for ~1 s more (same count on every
     # rank) so the clock / throttle record describes this workload
     for i in range(int(min(20000, max(0.0, 1000.0 / max(total_ms / args.steps, 1e-3))))):
@@ -595,6 +615,8 @@ def main():
         }
         if padded is not None:
             padded["segmented_over_padded"] = value / padded["value"]
+        if last is not None:
+            dump_outputs(args.dump_outputs, last[0], last[1], losses)
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,7 +1,7 @@
 """TEST / MEASUREMENT INFRASTRUCTURE ONLY.  Time the UNMODIFIED reference's PPO minibatch step on the host cores.
 
 Used by `bench.py --impl reference` and by bench.py's `cpu_baseline` leg when the reference is staged
-(`oracle/stage_ref.py` -> `oracle/_ref/`) or present at /root/reference.  The timed region is exactly the reference's
+(`oracle/stage_ref.py` -> `oracle/_ref/`).  The timed region is exactly the reference's
 minibatch body, urban_planning/agents/urban_planning_agent.py:327-337:
     tensorfy(states_b) -> value_loss -> ppo_entropy_loss -> loss.backward() -> clip_policy_grad -> optimizer.step
 with the reference's own modules (`create_sgnn_model`) and methods (`AgentPG.value_loss`,
@@ -26,7 +26,7 @@ class ReferenceStepper:
         from oracle import stage_ref
         root = stage_ref.staged_root()
         if root is None:
-            raise RuntimeError("the reference is neither staged (oracle/_ref) nor at /root/reference")
+            raise RuntimeError("the reference is not staged under oracle/_ref (oracle/stage_ref.py)")
         os.environ["UPB_REFERENCE_ROOT"] = root
         from oracle import ref_shim
         ref_shim.REFERENCE_ROOT = root

@@ -50,11 +50,10 @@ def stage(src_root: str = "/root/reference", dest: str = DEST) -> dict:
 
 
 def staged_root() -> str | None:
-    """Root to import the reference from: the staged copy, else the build container's /root/reference, else None."""
+    """Root to import the reference from: the copy staged under oracle/_ref, else None.  Run-time code reads only
+    this copy, never the tree it was staged from."""
     if os.path.isdir(os.path.join(DEST, "urban_planning")):
         return DEST
-    if os.path.isdir("/root/reference/urban_planning"):
-        return "/root/reference"
     return None
 
 
